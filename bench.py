@@ -7,6 +7,8 @@ the whole pipeline over one batch of 32 ragged utterances per GPU.
 
   python bench.py --gpus 1 --steps 3 --warmup 3            # ours (default)
   python bench.py --impl reference --steps 1 --warmup 0    # the reference's algorithm on the host CPU cores
+  python bench.py --dump-outputs DIR                       # also write the last timed step's waveforms to DIR/*.npy, so that
+                                                           # two builds can be compared output for output (same seeded inputs)
   torchrun --nnodes=1 --nproc-per-node N bench.py --gpus N ...   (N > 1: one rank per GPU; primary = the same 32 requests
                                                                    sharded over the ranks, "weak" key = 32 requests per rank)
 
@@ -191,6 +193,22 @@ def stage_roofline(stats, inputs, pk, nfe=10):
     return out
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, outputs, rank, world):
+    """--dump-outputs: what the last timed tts_batch_device call returned, as .npy files - wav (float32, the utterances' samples
+    back to back) and lens (float64, samples per utterance), with a _rank<r> suffix when several ranks run.  A waveform larger
+    than its rank's share of 64 MB is written as every k-th sample, k the smallest stride that fits."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    wav, lens = outputs["wav"].numpy(), outputs["lens"].numpy()
+    cap = (DUMP_BYTES // world - lens.nbytes) // wav.itemsize
+    np.save(os.path.join(path, f"wav{suffix}.npy"), wav[::max(1, -(-wav.size // cap))])
+    np.save(os.path.join(path, f"lens{suffix}.npy"), lens)
+
+
 # ================================================================================================ our arm (GPU)
 def run_ours(args):
     import torch
@@ -248,7 +266,7 @@ def run_ours(args):
         e0.record(model.stream)
         audio_s, stats = 0.0, None
         for _ in range(args.steps):
-            _, n, stats = model.tts_batch_device(inputs_dev)
+            wav, n, stats = model.tts_batch_device(inputs_dev)
             audio_s += sum(n) / 24000.0
         e1.record(model.stream)
         barrier()
@@ -257,6 +275,7 @@ def run_ours(args):
         launches = model.ctx.launch_count() - l0
         clocks = sampler.stop() if (rank == 0 and want_clocks) else None
         stats = model._stage_ms(stats)
+        outputs = dict(wav=wav.cpu(), lens=torch.tensor(n, dtype=torch.float64)) if args.dump_outputs else None
         # ---- timed region 2: end to end through the public API
         with torch.cuda.stream(model.stream):
             wav, n, _ = model.tts_batch_device(pinned)
@@ -285,7 +304,7 @@ def run_ours(args):
         dev_ms, e2e_ms, wall_ms = tt.tolist()
         audio_s, audio_e2e, launches, h2d_all = aa.tolist()
         return dict(value=audio_s / (dev_ms / 1000.0), e2e=audio_e2e / (e2e_ms / 1000.0), dev_ms=dev_ms, e2e_ms=e2e_ms, wall_ms=wall_ms,
-                    launches=int(launches), h2d=int(h2d_all), d2h=int(d2h), clocks=clocks, stats=stats, inputs=inputs)
+                    launches=int(launches), h2d=int(h2d_all), d2h=int(d2h), clocks=clocks, stats=stats, inputs=inputs, outputs=outputs)
 
     # ---- primary: the contract's split - the SAME `batch` utterances sharded over the ranks (strong scaling), LPT on expected tokens
     all_inputs = synth.batch32_zero_shot(batch)
@@ -299,6 +318,8 @@ def run_ours(args):
     model.ctx.profile(0)
     # ---- secondary: weak scaling (every rank its own `batch` requests)
     weak = measure(synth.batch32_zero_shot(batch, base=rank * batch), [batch] * world, False) if world > 1 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, strong["outputs"], rank, world)
     if rank != 0:
         if dist is not None:
             dist.destroy_process_group()
@@ -448,7 +469,12 @@ def main():
     ap.add_argument("--opt", action="append", default=[], help="library option key=value (cvk_set_option), repeatable")
     ap.add_argument("--workload", default="batch32", choices=["batch32", "cv3-bistream"],
                     help="batch32 = the headline metric (BASELINE.json configs[2]); cv3-bistream = configs[3] (1 GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="batch32 on the GPU: write the waveforms of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "batch32"):
+        ap.error("--dump-outputs applies to the batch32 workload of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "cv3-bistream":

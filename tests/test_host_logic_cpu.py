@@ -4,6 +4,7 @@ The text-streaming LM (llm.py:551-661) is mostly control flow (5:15 interleaving
 product implements it in Python over four C-ABI primitives.  Here those primitives are faked with the CPU oracle, so the
 host logic of `B200CosyVoice2Model.lm_generate_bistream` is checked against the reference's golden ids without a GPU.
 (The same method over the real library is checked by tests/test_lm_gpu.py::test_bistream_ids_match_reference_fp32.)"""
+import contextlib
 import threading
 
 import numpy as np
@@ -155,6 +156,11 @@ class _DummyEvent:
         pass
 
 
+def _dummy_stream_context(stream):
+    """torch.cuda.stream is a no-op only while no CUDA device is present; with one it would switch to the dummy stream"""
+    return contextlib.nullcontext()
+
+
 class FakeCtx3:
     """the libcvk calls B200CosyVoice3Model makes (batched LM session API, flow3, hift3) on the CPU oracles"""
 
@@ -249,6 +255,7 @@ def test_cosyvoice3_model_host_glue_matches_reference(golden, monkeypatch):
     from cosyvoice_b200.model3 import B200CosyVoice3Model
     from oracle import dit, hift_causal as hc, weights
     monkeypatch.setattr(torch.cuda, "Event", _DummyEvent)
+    monkeypatch.setattr(torch.cuda, "stream", _dummy_stream_context)
     g = golden("stream3_tts")
     text, ptext, ptok, U = cases.lm3_case()
     _, _, pfeat, emb = cases.flow_case(P=9)
@@ -345,6 +352,7 @@ def test_cosyvoice2_model_host_glue_matches_reference(golden, monkeypatch):
     from oracle import flow, hift, weights
     from oracle.make_golden import stream_noise
     monkeypatch.setattr(torch.cuda, "Event", _DummyEvent)
+    monkeypatch.setattr(torch.cuda, "stream", _dummy_stream_context)
     g = golden("stream_tts")
     text, ptext, ptok, U = cases.lm_case()
     _, _, pfeat, emb = cases.flow_case(P=9)

@@ -1,6 +1,7 @@
 """GPU: parity of the BENCHMARKED mode (bf16 tensor-core operands, persistent LM decode kernel) at the BENCHMARK shape - one
 full-size Z10 utterance (24-layer LM over 389 positions, 325 tokens -> 650 mel frames through the full flow, 500 frames through the
-vocoder) against the CPU oracle's outputs committed in tests/golden/z10_full.npz (oracle/make_golden_full.py).
+vocoder) against the CPU oracle's outputs committed in tests/golden/z10_full.npz (oracle/make_golden_full.py; the vocoder's source
+and waveform are recomputed from the committed mel and checked against committed samples).
 
 SURVEY.md §8(c)(iii) protocol: teacher-forced log-probs (max |d| and top-25 set overlap), mel after 10 Euler steps against fp32 with
 the reference-style 16-bit autocast deviation printed beside it as the yardstick, waveform with the source injected.  Every test
@@ -11,7 +12,7 @@ import torch
 
 from gpu_util import maxdiff
 from oracle import flow, hift, lm, weights
-from oracle.make_golden_full import LM_ROWS, case
+from oracle.make_golden_full import LM_ROWS, PIN_STRIDE, case
 
 pytestmark = pytest.mark.gpu
 _c = {}
@@ -119,11 +120,17 @@ def test_hift_wav_fullsize(golden):
     c = bctx()
     sd = weights.synth_state_dict(hift.param_shapes(), 1986, hift.SYNTH_GAINS)
     c.load_state_dict("hift", sd)
-    mel_tm = torch.from_numpy(g["mel"])[0].t().contiguous()
+    mel = torch.from_numpy(g["mel"])
+    # the oracle's source and waveform for the committed mel, recomputed on the CPU from the seeded noise and pinned to the
+    # committed samples (make_golden_full.py stores every PIN_STRIDE-th one)
+    wav_ref, src = hift.inference(sd, mel, case()[2])
+    src, ref = src.reshape(-1), wav_ref.reshape(-1)
+    assert np.abs(src[::PIN_STRIDE].numpy() - g["source_pin"]).max() < 1e-4
+    assert np.abs(ref[::PIN_STRIDE].numpy() - g["wav_pin"]).max() < 1e-4
+    mel_tm = mel[0].t().contiguous()
     f0 = c.hift_f0(mel_tm, [500]).cpu()
     print(f"[full-size vocoder] f0 max |d| {(f0 - torch.from_numpy(g['f0']).reshape(-1)).abs().max().item():.4g} Hz")
-    wav = c.hift_decode(mel_tm, [500], torch.from_numpy(g["source"]).reshape(-1)).cpu()
-    ref = torch.from_numpy(g["wav"]).reshape(-1)
+    wav = c.hift_decode(mel_tm, [500], src).cpu()
     d = (wav - ref).abs()
     snr = 10 * torch.log10(ref.pow(2).sum() / (wav - ref).pow(2).sum()).item()
     print(f"[full-size vocoder, ctx precision bf16] wav max |d| {d.max().item():.4g}, rms {d.pow(2).mean().sqrt().item():.4g} on |wav| <= {ref.abs().max().item():.3g}; SNR {snr:.1f} dB")
