@@ -11,8 +11,10 @@ normalisation, no tokenizer (those stay with the reference's frontend and server
 Admission policy: a batch is closed when ``max_batch`` requests are waiting or ``max_wait_ms`` have passed since the first one
 arrived; requests are never reordered inside a batch (the model's RNG streams are consumed in input order, so a fixed arrival
 order gives fixed results).  One worker thread owns the model; ``tts_batch`` itself is ragged, so no padding or bucketing is
-needed here.
+needed here.  Streaming requests (``submit_stream``) share the queue: a closed batch serves its streaming requests through one
+``tts_stream_batch`` and its offline requests through one ``tts_batch``.  A request never joins a batch that is already running.
 """
+import queue
 import threading
 import time
 from concurrent.futures import Future
@@ -34,6 +36,35 @@ def pcm16_decode(buf):
     (runtime/python/grpc/server.py:45-46: ``np.frombuffer(..., dtype=np.int16)`` then ``.float() / (2 ** 15)``)."""
     import torch
     return torch.from_numpy(np.array(np.frombuffer(buf, dtype=np.int16))).unsqueeze(0).float() / (2 ** 15)
+
+
+class ChunkStream:
+    """Iterator over one streaming request's chunks, fed by the batcher's worker: [1, n] float32 CPU tensors, or int16 PCM bytes
+    for ``submit_stream_pcm``.  Ends after the request's last chunk; raises the batch's exception if its batch failed."""
+
+    def __init__(self, pcm):
+        self.pcm = pcm
+        self._q = queue.Queue()
+        self._end = None
+
+    def _put(self, wave):
+        self._q.put((0, pcm16(wave) if self.pcm else wave))
+
+    def _finish(self, exc=None):
+        self._q.put((1, exc))
+
+    def __iter__(self):
+        return self
+
+    def __next__(self):
+        if self._end is None:
+            kind, v = self._q.get()
+            if kind == 0:
+                return v
+            self._end = (v,)
+        if self._end[0] is not None:
+            raise self._end[0]
+        raise StopIteration
 
 
 class TtsBatcher:
@@ -61,14 +92,22 @@ class TtsBatcher:
     def submit_pcm(self, **request):
         return self._enqueue(request, True)
 
-    def _enqueue(self, request, pcm):
-        fut = Future()
+    def submit_stream(self, **request):
+        """-> iterator of the request's chunks ([1, n] float32 CPU tensors, what ``tts(stream=True)`` yields for it alone)"""
+        return self._enqueue(request, False, ChunkStream(False))
+
+    def submit_stream_pcm(self, **request):
+        """-> iterator of the request's chunks as int16 PCM bytes (the reference servers' per-chunk wire format)"""
+        return self._enqueue(request, True, ChunkStream(True))
+
+    def _enqueue(self, request, pcm, sink=None):
+        sink = sink if sink is not None else Future()
         with self._cv:
             if self._closed:
                 raise RuntimeError("TtsBatcher is closed")
-            self._q.append((request, fut, pcm, time.monotonic()))
+            self._q.append((request, sink, pcm, time.monotonic()))
             self._cv.notify_all()
-        return fut
+        return sink
 
     def close(self, wait=True):
         """Stop admitting; requests already queued are still served."""
@@ -105,18 +144,43 @@ class TtsBatcher:
             batch = self._take_batch()
             if batch is None:
                 return
-            live = [b for b in batch if b[1].set_running_or_notify_cancel()]
+            live = [b for b in batch if isinstance(b[1], ChunkStream) or b[1].set_running_or_notify_cancel()]
             if not live:
                 continue
             self.batches.append(len(live))
+            streams = [b for b in live if isinstance(b[1], ChunkStream)]
+            offline = [b for b in live if not isinstance(b[1], ChunkStream)]
+            # the kind that arrived first is served first
+            for group in sorted((g for g in (streams, offline) if g), key=lambda g: g[0][3]):
+                if group is streams:
+                    self._serve_streams(streams)
+                else:
+                    self._serve_offline(offline)
+
+    def _serve_offline(self, live):
+        try:
+            waves = self.model.tts_batch([b[0] for b in live])
+        except BaseException as e:          # the whole batch shares the failure (one launch sequence)
+            for _, fut, _, _ in live:
+                fut.set_exception(e)
+            return
+        for (_, fut, pcm, _), w in zip(live, waves):
             try:
-                waves = self.model.tts_batch([b[0] for b in live])
-            except BaseException as e:          # the whole batch shares the failure (one launch sequence)
-                for _, fut, _, _ in live:
-                    fut.set_exception(e)
-                continue
-            for (_, fut, pcm, _), w in zip(live, waves):
-                try:
-                    fut.set_result(pcm16(w) if pcm else w)
-                except BaseException as e:
-                    fut.set_exception(e)
+                fut.set_result(pcm16(w) if pcm else w)
+            except BaseException as e:
+                fut.set_exception(e)
+
+    def _serve_streams(self, live):
+        open_ = set(range(len(live)))
+        try:
+            for i, out, last in self.model.tts_stream_batch([b[0] for b in live]):
+                live[i][1]._put(out["tts_speech"])
+                if last:
+                    live[i][1]._finish()
+                    open_.discard(i)
+        except BaseException as e:          # the failure reaches every request of this batch that has not ended
+            for i in sorted(open_):
+                live[i][1]._finish(e)
+            return
+        for i in sorted(open_):
+            live[i][1]._finish(RuntimeError("tts_stream_batch ended without the request's last chunk"))

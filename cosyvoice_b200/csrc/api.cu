@@ -398,35 +398,45 @@ int cvk_flow_inference(cvk_ctx* ctx, const int32_t* tokens, const int* token_len
                  (cudaStream_t)stream);
   CVK_API_END
 }
-int cvk_flow_stream_create(cvk_ctx* ctx, int max_frames, int n_timesteps, cvk_flow_stream** out) {
+int cvk_flow_stream_slots_create(cvk_ctx* ctx, int kind, int n_slots, int max_frames, int n_timesteps, cvk_flow_stream** out) {
   CVK_API_BEGIN
-  CVK_REQUIRE(out != nullptr, "cvk_flow_stream_create: bad arguments");
-  *out = flow_stream_create(ctx, max_frames, n_timesteps, 0);
+  CVK_REQUIRE(out != nullptr, "cvk_flow_stream_slots_create: bad arguments");
+  *out = flow_stream_create(ctx, kind, n_slots, max_frames, n_timesteps);
   CVK_API_END
 }
+int cvk_flow_stream_create(cvk_ctx* ctx, int max_frames, int n_timesteps, cvk_flow_stream** out) {
+  return cvk_flow_stream_slots_create(ctx, 0, 1, max_frames, n_timesteps, out);
+}
 int cvk_flow3_stream_create(cvk_ctx* ctx, int max_frames, int n_timesteps, cvk_flow_stream** out) {
-  CVK_API_BEGIN
-  CVK_REQUIRE(out != nullptr, "cvk_flow3_stream_create: bad arguments");
-  *out = flow_stream_create(ctx, max_frames, n_timesteps, 1);
-  CVK_API_END
+  return cvk_flow_stream_slots_create(ctx, 1, 1, max_frames, n_timesteps, out);
 }
 void cvk_flow_stream_destroy(cvk_ctx* ctx, cvk_flow_stream* fs) {
   if (!ctx || !fs) return;
   try { cudaSetDevice(ctx->device); flow_stream_destroy(fs); } catch (...) {}
 }
 long long cvk_flow_stream_bytes(const cvk_flow_stream* fs) { return fs ? (long long)flow_stream_bytes(fs) : 0; }
-int cvk_flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, const float* prompt_feat, int prompt_frames, const float* embedding, void* stream) {
+int cvk_flow_stream_slot_begin(cvk_ctx* ctx, cvk_flow_stream* fs, int slot, const float* prompt_feat, int prompt_frames, const float* embedding,
+                               void* stream) {
   CVK_API_BEGIN
-  CVK_REQUIRE(fs && embedding && (prompt_feat || prompt_frames == 0), "cvk_flow_stream_begin: bad arguments");
-  flow_stream_begin(ctx, fs, prompt_feat, prompt_frames, embedding, (cudaStream_t)stream);
+  CVK_REQUIRE(fs && embedding && (prompt_feat || prompt_frames == 0), "cvk_flow_stream_slot_begin: bad arguments");
+  flow_stream_begin(ctx, fs, slot, prompt_feat, prompt_frames, embedding, (cudaStream_t)stream);
+  CVK_API_END
+}
+int cvk_flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, const float* prompt_feat, int prompt_frames, const float* embedding, void* stream) {
+  return cvk_flow_stream_slot_begin(ctx, fs, 0, prompt_feat, prompt_frames, embedding, stream);
+}
+int cvk_flow_stream_chunk_batch(cvk_ctx* ctx, cvk_flow_stream* fs, int B, const int* slots_host, const int32_t* tokens,
+                                const int* token_lens_host, float* mel_out, int mel_capacity_frames, int* n_frames_out_host, void* stream) {
+  CVK_API_BEGIN
+  CVK_REQUIRE(fs && B > 0 && slots_host && tokens && token_lens_host && mel_out && n_frames_out_host, "cvk_flow_stream_chunk_batch: bad arguments");
+  for (int b = 0; b < B; ++b) CVK_REQUIRE(token_lens_host[b] > 3, "cvk_flow_stream_chunk_batch: a prefix without its 3 look-ahead tokens");
+  flow_stream_chunk_batch(ctx, fs, B, slots_host, tokens, token_lens_host, mel_out, mel_capacity_frames, n_frames_out_host, (cudaStream_t)stream);
   CVK_API_END
 }
 int cvk_flow_stream_chunk(cvk_ctx* ctx, cvk_flow_stream* fs, const int32_t* tokens, int n_tokens, float* mel_out, int mel_capacity_frames,
                           int* n_frames_out, void* stream) {
-  CVK_API_BEGIN
-  CVK_REQUIRE(fs && tokens && mel_out && n_frames_out && n_tokens > 3, "cvk_flow_stream_chunk: bad arguments");
-  *n_frames_out = flow_stream_chunk(ctx, fs, tokens, n_tokens, mel_out, mel_capacity_frames, (cudaStream_t)stream);
-  CVK_API_END
+  const int slot = 0;
+  return cvk_flow_stream_chunk_batch(ctx, fs, 1, &slot, tokens, &n_tokens, mel_out, mel_capacity_frames, n_frames_out, stream);
 }
 int cvk_cfm_set_noise(cvk_ctx* ctx, const float* noise_tm, int T, int on_device) {
   CVK_API_BEGIN

@@ -298,11 +298,13 @@ void whisper_log_mel(cvk_ctx* ctx, const float* wav, const int* lens, int B, flo
 void kaldi_fbank80(cvk_ctx* ctx, const float* wav, const int* lens, int B, int subtract_mean, float* out, cudaStream_t st);
 // incremental streaming flow (flow.cu)
 struct cvk_flow_stream;
-cvk_flow_stream* flow_stream_create(cvk_ctx* ctx, int max_frames, int n_timesteps, int kind);
+cvk_flow_stream* flow_stream_create(cvk_ctx* ctx, int kind, int n_slots, int max_frames, int n_timesteps);
 void flow_stream_destroy(cvk_flow_stream* fs);
 size_t flow_stream_bytes(const cvk_flow_stream* fs);
-void flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, const float* prompt_feat, int prompt_frames, const float* embedding, cudaStream_t st);
-int flow_stream_chunk(cvk_ctx* ctx, cvk_flow_stream* fs, const int32_t* tokens, int n_tokens, float* mel_out, int mel_cap_frames, cudaStream_t st);
+void flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, int slot, const float* prompt_feat, int prompt_frames, const float* embedding,
+                       cudaStream_t st);
+void flow_stream_chunk_batch(cvk_ctx* ctx, cvk_flow_stream* fs, int B, const int* slots, const int32_t* tokens, const int* token_lens,
+                             float* mel_out, int mel_cap_frames, int* n_out, cudaStream_t st);
 void attention_fwd(cvk_ctx* ctx, cudaStream_t st, const Mat& q, const Mat& k, const Mat& v, const Seqs& s, int H, int chunk,
                    float scale, const Mat& out, int kv_div = 1, const KvGeom* kg = nullptr);
 void relpos_attention_fwd(cvk_ctx* ctx, cudaStream_t st, const Mat& q, const Mat& k, const Mat& v, const Mat& pos /*[2*Tmax-1, H*64]*/,

@@ -58,25 +58,26 @@ struct FlowModel {
   int noise_T = 0;
 };
 
-// One streaming synthesis session of the flow stage (cvk_flow_stream_*): the caches that let a chunk call compute ONLY its
-// new frames.  Per Euler step: K/V rows of every estimator transformer block for both CFG sequences, and the two-row tails of
-// every causal convolution's input.
+// Streaming synthesis sessions of the flow stage (cvk_flow_stream_*): the caches that let a chunk call compute ONLY its new
+// frames, for n_slots utterances in one allocation.  Per Euler step: K/V rows of every estimator transformer block for both CFG
+// sequences of every slot (slot s, branch c at rows (2s + c) * cap), and the tails of every causal convolution's input.
 struct cvk_flow_stream {
   int kind = 0;                 // 0: CosyVoice2 U-Net estimator (stage "flow"), 1: CosyVoice3 DiT (stage "flow3")
   int kv_width = 1024;          // K | V columns per cached row: 2 x 512 (U-Net blocks), 2 x 1024 (DiT blocks)
   int tail_rows = 2;            // rows a causal convolution reads in front of a chunk: k3 -> 2, the DiT's k31 position convolutions -> 30
   int conv_c = 512;             // widest convolution input
-  int cap = 0, n_steps = 0, adt = DT_F32, n_tb = 0, n_conv = 0;
-  void* kv = nullptr;
-  void* conv = nullptr;
+  int cap = 0, n_slots = 1, n_steps = 0, adt = DT_F32, n_tb = 0, n_conv = 0;
+  void* kv = nullptr;           // per step: [n_tb][n_slots * 2 * cap + 64][kv_width]
+  void* conv = nullptr;         // per step: [n_conv][n_slots * 2][tail_rows][conv_c]
   size_t kv_step_bytes = 0, conv_step_bytes = 0;
-  int frames_done = 0;          // mel frames (prompt included) already produced
-  int prompt_frames = 0;
-  float* prompt_feat = nullptr; // [prompt_frames][80]
-  float* spk = nullptr;         // [80] projected speaker embedding
-  int* d_geo = nullptr;         // kstart[2] | klen[2] | qoff[2]
+  std::vector<int> frames_done; // per slot: mel frames (prompt included) already produced
+  std::vector<int> prompt_frames;
+  std::vector<char> begun;
+  float* prompt_feat = nullptr; // [n_slots][cap][80]
+  float* spk = nullptr;         // [n_slots][80] projected speaker embeddings
+  int* d_geo = nullptr;         // per sequence of a call (2 per slot): kstart | klen | qoff | conv state index, 2 * n_slots each
   KvGeom kg;
-  bool begun = false;
+  const int* d_cidx = nullptr;
 };
 
 namespace {
@@ -573,22 +574,22 @@ struct EstBuffers {
 // convolution the last two input rows, are all a later call needs.  The reference recomputes the prefix instead
 // (cli/model.py:346-363).
 struct EstInc {
-  void* kv = nullptr;        // [n_tblocks][2 * cap + 64][kv_width] act dtype: K | V rows of CFG sequence 0 then 1
-  void* conv = nullptr;      // [n_convs][2 seqs][tail_rows][conv_c] act dtype
+  void* kv = nullptr;        // [n_tblocks][kv_rows][kv_width] act dtype: K | V rows, sequence b's from row kg.d_kstart[b]
+  void* conv = nullptr;      // [n_convs][n_states][tail_rows][conv_c] act dtype, sequence b's tail at state cidx[b]
   int kv_width = 1024, tail_rows = 2, conv_c = 512;
-  int cap = 0;               // cache rows per sequence
-  int t_prev = 0;            // frames already cached
+  int kv_rows = 0, n_states = 0;
   int tb_idx = 0, conv_idx = 0;
   KvGeom kg;
+  const int* d_cidx = nullptr;
 };
 
 template <typename T>
 __global__ void conv_state_kernel(T* __restrict__ x, int ld, int C, const int* __restrict__ start, const int* __restrict__ len, T* __restrict__ state,
-                                  int tail, int cstride) {
+                                  int tail, int cstride, const int* __restrict__ cidx) {
   // gap rows start-tail .. start-1 <- saved tail of the previous chunk; saved tail <- last `tail` rows of this chunk (chunks are at
   // least 50 rows, so the two row ranges never overlap)
   const int b = blockIdx.x, r = blockIdx.y;
-  T* srow = state + ((size_t)b * tail + r) * cstride;
+  T* srow = state + ((size_t)cidx[b] * tail + r) * cstride;
   T* gap = x + (size_t)(start[b] - tail + r) * ld;
   const T* tl = x + (size_t)(start[b] + len[b] - tail + r) * ld;
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
@@ -598,30 +599,57 @@ __global__ void conv_state_kernel(T* __restrict__ x, int ld, int C, const int* _
 }
 
 // rows of a chunk's K | V columns (qkv columns [koff, koff + width)) appended to the cache of its sequence; the chunk's first row
-// goes to cache row qoff[b] (device memory, so that a captured launch stays valid from chunk to chunk)
+// goes to cache row kstart[b] + qoff[b] (device memory, so that a captured launch stays valid from chunk to chunk)
 template <typename T>
 __global__ void kv_append_kernel(const T* __restrict__ qkv, int ld, int koff, int width, const int* __restrict__ start, const int* __restrict__ len,
-                                 T* __restrict__ cache, int cap, const int* __restrict__ qoff) {
+                                 T* __restrict__ cache, const int* __restrict__ kstart, const int* __restrict__ qoff) {
   const int b = blockIdx.y;
-  const int L = len[b], t_prev = qoff[b];
+  const int L = len[b], row0 = kstart[b] + qoff[b];
   for (int i = blockIdx.x; i < L; i += gridDim.x) {
     const uint4* src = reinterpret_cast<const uint4*>(qkv + (size_t)(start[b] + i) * ld + koff);
-    uint4* dst = reinterpret_cast<uint4*>(cache + ((size_t)b * cap + t_prev + i) * width);
+    uint4* dst = reinterpret_cast<uint4*>(cache + ((size_t)row0 + i) * width);
     for (int c = threadIdx.x; c < width * (int)sizeof(T) / 16; c += blockDim.x) dst[c] = src[c];
+  }
+}
+
+// inputs of one multi-slot chunk call: sequence b (slot slot[b], frames [t_prev[b], t_prev[b] + len1[b])) gets its new rows of mu
+// (mu_full, geometry start2), of the CFM noise, and of its slot's prompt conditioning (zero past pfr[b]) in geometry start1, and
+// its slot's speaker row in spk_out[b]
+__global__ void stream_gather_kernel(const float* __restrict__ mu_full, const int* __restrict__ start2, const float* __restrict__ noise,
+                                     const float* __restrict__ prompt_feat, const float* __restrict__ spk, int cap,
+                                     const int* __restrict__ geo /*t_prev[B] | pfr[B] | slot[B]*/, int B, const int* __restrict__ start1,
+                                     const int* __restrict__ len1, float* __restrict__ mu, float* __restrict__ cond, float* __restrict__ x,
+                                     float* __restrict__ spk_out) {
+  const int b = blockIdx.y;
+  const int t_prev = geo[b], pfr = geo[B + b], slot = geo[2 * B + b], L = len1[b];
+  if (blockIdx.x == 0)
+    for (int c = threadIdx.x; c < N_MEL; c += blockDim.x) spk_out[(size_t)b * N_MEL + c] = spk[(size_t)slot * N_MEL + c];
+  for (int t = blockIdx.x; t < L; t += gridDim.x) {
+    const int g = t_prev + t;
+    const size_t r1 = (size_t)(start1[b] + t) * N_MEL;
+    const float* m = mu_full + (size_t)(start2[b] + g) * N_MEL;
+    const float* pf = prompt_feat + ((size_t)slot * cap + g) * N_MEL;
+    for (int c = threadIdx.x; c < N_MEL; c += blockDim.x) {
+      mu[r1 + c] = m[c];
+      x[r1 + c] = noise[(size_t)g * N_MEL + c];
+      cond[r1 + c] = g < pfr ? pf[c] : 0.f;
+    }
   }
 }
 
 // the two rows a causal k=3 convolution reads in front of the chunk (call right before the convolution that consumes `in`)
 void conv_state(cvk_ctx* ctx, cudaStream_t st, EstInc* inc, const Mat& in, const Seqs& s) {
   if (!inc) return;
-  CVK_REQUIRE(in.cols <= inc->conv_c && s.B == 2, "conv_state: unexpected operand");
+  CVK_REQUIRE(in.cols <= inc->conv_c && s.B <= inc->n_states, "conv_state: unexpected operand");
   const size_t es = in.esize();
-  char* state = (char*)inc->conv + (size_t)inc->conv_idx * 2 * inc->tail_rows * inc->conv_c * es;
+  char* state = (char*)inc->conv + (size_t)inc->conv_idx * inc->n_states * inc->tail_rows * inc->conv_c * es;
   ++inc->conv_idx;
   if (in.dtype == DT_F32)
-    conv_state_kernel<float><<<dim3(s.B, inc->tail_rows), 128, 0, st>>>(in.f32(), in.ld, in.cols, s.d_start, s.d_len, (float*)state, inc->tail_rows, inc->conv_c);
+    conv_state_kernel<float><<<dim3(s.B, inc->tail_rows), 128, 0, st>>>(in.f32(), in.ld, in.cols, s.d_start, s.d_len, (float*)state, inc->tail_rows, inc->conv_c,
+                                                                        inc->d_cidx);
   else
-    conv_state_kernel<bf16><<<dim3(s.B, inc->tail_rows), 128, 0, st>>>(in.b16(), in.ld, in.cols, s.d_start, s.d_len, (bf16*)state, inc->tail_rows, inc->conv_c);
+    conv_state_kernel<bf16><<<dim3(s.B, inc->tail_rows), 128, 0, st>>>(in.b16(), in.ld, in.cols, s.d_start, s.d_len, (bf16*)state, inc->tail_rows, inc->conv_c,
+                                                                       inc->d_cidx);
   ctx->launches++;
   CVK_LAUNCH_CHECK();
 }
@@ -629,14 +657,16 @@ void conv_state(cvk_ctx* ctx, cudaStream_t st, EstInc* inc, const Mat& in, const
 // append the chunk's K | V rows (columns [koff, koff + kv_width) of qkv) to the cache of the next block and return that cache
 Mat kv_cache_append(cvk_ctx* ctx, cudaStream_t st, EstInc* inc, const Mat& qkv, int koff, const Seqs& s) {
   const size_t es = qkv.esize();
-  const int crow = 2 * inc->cap + 64;
+  const int crow = inc->kv_rows;
   Mat cache((char*)inc->kv + (size_t)inc->tb_idx * crow * inc->kv_width * es, qkv.dtype, crow, inc->kv_width, inc->kv_width);
   ++inc->tb_idx;
   int bx = s.max_len < 256 ? s.max_len : 256;
   if (qkv.dtype == DT_F32)
-    kv_append_kernel<float><<<dim3(bx, s.B), 128, 0, st>>>(qkv.f32(), qkv.ld, koff, inc->kv_width, s.d_start, s.d_len, cache.f32(), inc->cap, inc->kg.d_qoff);
+    kv_append_kernel<float><<<dim3(bx, s.B), 128, 0, st>>>(qkv.f32(), qkv.ld, koff, inc->kv_width, s.d_start, s.d_len, cache.f32(), inc->kg.d_kstart,
+                                                           inc->kg.d_qoff);
   else
-    kv_append_kernel<bf16><<<dim3(bx, s.B), 128, 0, st>>>(qkv.b16(), qkv.ld, koff, inc->kv_width, s.d_start, s.d_len, cache.b16(), inc->cap, inc->kg.d_qoff);
+    kv_append_kernel<bf16><<<dim3(bx, s.B), 128, 0, st>>>(qkv.b16(), qkv.ld, koff, inc->kv_width, s.d_start, s.d_len, cache.b16(), inc->kg.d_kstart,
+                                                          inc->kg.d_qoff);
   ctx->launches++;
   CVK_LAUNCH_CHECK();
   return cache;
@@ -843,9 +873,10 @@ void cfm_solve_packed(cvk_ctx* ctx, cudaStream_t st, const Seqs& s1, const int* 
       EstInc inc;
       inc.kv = (char*)fs->kv + (size_t)step * fs->kv_step_bytes;
       inc.conv = (char*)fs->conv + (size_t)step * fs->conv_step_bytes;
-      inc.cap = fs->cap;
-      inc.t_prev = fs->frames_done;
+      inc.kv_rows = 2 * fs->n_slots * fs->cap + 64;
+      inc.n_states = 2 * fs->n_slots;
       inc.kg = fs->kg;
+      inc.d_cidx = fs->d_cidx;
       inc.kv_width = fs->kv_width; inc.tail_rows = fs->tail_rows; inc.conv_c = fs->conv_c;
       if (dit) dit_estimator_forward(ctx, st, s2, in0, t_dev + (size_t)step * 2 * B, streaming, v, &inc);
       else estimator_forward(ctx, st, s2, in0, t_dev + (size_t)step * 2 * B, streaming, v, &inc);
@@ -1257,15 +1288,20 @@ void flow_inference(cvk_ctx* ctx, const int32_t* tokens, const int* token_lens, 
 static Mat dit_mu_forward(cvk_ctx* ctx, cudaStream_t st, const int32_t* tokens, const int* token_lens, int B, int ctxl, Seqs* s2_out);
 void flow_stream_destroy(cvk_flow_stream* fs);
 
-// kind 0: CosyVoice2 U-Net estimator (stage "flow"); kind 1: CosyVoice3 DiT (stage "flow3")
-cvk_flow_stream* flow_stream_create(cvk_ctx* ctx, int max_frames, int n_timesteps, int kind) {
+// kind 0: CosyVoice2 U-Net estimator (stage "flow"); kind 1: CosyVoice3 DiT (stage "flow3").  n_slots utterances share the
+// allocation; the reference gives every streaming request its own thread and recomputes its prefix (cli/model.py:343-363).
+cvk_flow_stream* flow_stream_create(cvk_ctx* ctx, int kind, int n_slots, int max_frames, int n_timesteps) {
   CVK_REQUIRE(kind == 0 || kind == 1, "flow stream: unknown estimator kind");
-  CVK_REQUIRE(max_frames >= 2 * CHUNK_TOK && n_timesteps >= 1, "flow stream: bad capacity / step count");
+  CVK_REQUIRE(n_slots >= 1 && max_frames >= 2 * CHUNK_TOK && n_timesteps >= 1, "flow stream: bad slot count / capacity / step count");
   cvk_flow_stream* fs = new cvk_flow_stream();
   fs->kind = kind;
   fs->cap = round_up(max_frames, 64);
+  fs->n_slots = n_slots;
   fs->n_steps = n_timesteps;
   fs->adt = ctx->act_dtype;
+  fs->frames_done.assign(n_slots, 0);
+  fs->prompt_frames.assign(n_slots, 0);
+  fs->begun.assign(n_slots, 0);
   const size_t es = fs->adt == DT_F32 ? 4 : 2;
   if (kind == 0) {
     FlowModel* m = ctx->flow;
@@ -1281,14 +1317,14 @@ cvk_flow_stream* flow_stream_create(cvk_ctx* ctx, int max_frames, int n_timestep
     fs->n_conv = 2;                   // the two grouped k31 position convolutions of the input embedding
     fs->kv_width = 2 * DIT_D; fs->tail_rows = DIT_CK - 1; fs->conv_c = DIT_D;
   }
-  fs->kv_step_bytes = (size_t)fs->n_tb * (2 * fs->cap + 64) * fs->kv_width * es;
-  fs->conv_step_bytes = (size_t)fs->n_conv * 2 * fs->tail_rows * fs->conv_c * es;
+  fs->kv_step_bytes = (size_t)fs->n_tb * ((size_t)2 * n_slots * fs->cap + 64) * fs->kv_width * es;
+  fs->conv_step_bytes = (size_t)fs->n_conv * 2 * n_slots * fs->tail_rows * fs->conv_c * es;
   try {
     CVK_CHECK_CUDA(cudaMalloc(&fs->kv, fs->kv_step_bytes * n_timesteps));
     CVK_CHECK_CUDA(cudaMalloc(&fs->conv, fs->conv_step_bytes * n_timesteps));
-    CVK_CHECK_CUDA(cudaMalloc(&fs->prompt_feat, sizeof(float) * (size_t)fs->cap * N_MEL));
-    CVK_CHECK_CUDA(cudaMalloc(&fs->spk, sizeof(float) * N_MEL));
-    CVK_CHECK_CUDA(cudaMalloc(&fs->d_geo, sizeof(int) * 6));
+    CVK_CHECK_CUDA(cudaMalloc(&fs->prompt_feat, sizeof(float) * (size_t)n_slots * fs->cap * N_MEL));
+    CVK_CHECK_CUDA(cudaMalloc(&fs->spk, sizeof(float) * (size_t)n_slots * N_MEL));
+    CVK_CHECK_CUDA(cudaMalloc(&fs->d_geo, sizeof(int) * 8 * n_slots));
     CVK_CHECK_CUDA(cudaMemset(fs->kv, 0, fs->kv_step_bytes * n_timesteps));   // masked key rows of a partial tile must be finite
   } catch (...) {                      // out of memory half way: give back what was taken
     cudaGetLastError();
@@ -1296,8 +1332,9 @@ cvk_flow_stream* flow_stream_create(cvk_ctx* ctx, int max_frames, int n_timestep
     throw;
   }
   fs->kg.d_kstart = fs->d_geo;
-  fs->kg.d_klen = fs->d_geo + 2;
-  fs->kg.d_qoff = fs->d_geo + 4;
+  fs->kg.d_klen = fs->d_geo + 2 * n_slots;
+  fs->kg.d_qoff = fs->d_geo + 4 * n_slots;
+  fs->d_cidx = fs->d_geo + 6 * n_slots;
   return fs;
 }
 
@@ -1309,57 +1346,82 @@ void flow_stream_destroy(cvk_flow_stream* fs) {
 
 size_t flow_stream_bytes(const cvk_flow_stream* fs) { return (fs->kv_step_bytes + fs->conv_step_bytes) * (size_t)fs->n_steps; }
 
-// new utterance: prompt mel [prompt_frames][80] and speaker embedding [192] (device pointers); clears the caches
-void flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, const float* prompt_feat, int prompt_frames, const float* embedding, cudaStream_t st) {
+static void require_stage(cvk_ctx* ctx, const cvk_flow_stream* fs) {
   CVK_REQUIRE(fs->kind == 0 ? (ctx->flow && ctx->flow->tok_emb) : (ctx->dit && ctx->dit->tok_emb), "flow stage of this session not finalised");
-  const ConvW& spk_affine = fs->kind == 0 ? ctx->flow->spk_affine : ctx->dit->spk_affine;
   CVK_REQUIRE(fs->adt == ctx->act_dtype, "flow stream was created under another precision");
+}
+
+// new utterance in `slot`: prompt mel [prompt_frames][80] and speaker embedding [192] (device pointers); clears the slot's
+// convolution tails (its K/V rows are overwritten chunk by chunk and never read beyond what was written)
+void flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, int slot, const float* prompt_feat, int prompt_frames, const float* embedding, cudaStream_t st) {
+  require_stage(ctx, fs);
+  const ConvW& spk_affine = fs->kind == 0 ? ctx->flow->spk_affine : ctx->dit->spk_affine;
+  CVK_REQUIRE(slot >= 0 && slot < fs->n_slots, "flow stream: slot out of range");
   CVK_REQUIRE(prompt_frames >= 0 && prompt_frames < fs->cap, "flow stream: prompt longer than the cache");
   ctx->arena.reset();
-  CVK_CHECK_CUDA(cudaMemsetAsync(fs->conv, 0, fs->conv_step_bytes * fs->n_steps, st));    // causal left padding of the first chunk
+  // causal left padding of the first chunk: the slot's 2 states of every (step, convolution), one pitched row each
+  const size_t es = fs->adt == DT_F32 ? 4 : 2;
+  const size_t state_bytes = (size_t)fs->tail_rows * fs->conv_c * es;
+  CVK_CHECK_CUDA(cudaMemset2DAsync((char*)fs->conv + (size_t)2 * slot * state_bytes, (size_t)2 * fs->n_slots * state_bytes, 0, 2 * state_bytes,
+                                   (size_t)fs->n_steps * fs->n_conv, st));
   if (prompt_frames > 0)
-    CVK_CHECK_CUDA(cudaMemcpyAsync(fs->prompt_feat, prompt_feat, sizeof(float) * (size_t)prompt_frames * N_MEL, cudaMemcpyDeviceToDevice, st));
+    CVK_CHECK_CUDA(cudaMemcpyAsync(fs->prompt_feat + (size_t)slot * fs->cap * N_MEL, prompt_feat, sizeof(float) * (size_t)prompt_frames * N_MEL,
+                                   cudaMemcpyDeviceToDevice, st));
   Mat en = arena_mat(ctx, DT_F32, 1, 192);
   l2norm_kernel<<<1, 64, 0, st>>>(embedding, en.f32(), 192);
   ctx->launches++;
   CVK_LAUNCH_CHECK();
   {
     Epilogue e;
-    e.out = Mat(fs->spk, DT_F32, 1, N_MEL, N_MEL);
+    e.out = Mat(fs->spk + (size_t)slot * N_MEL, DT_F32, 1, N_MEL, N_MEL);
     conv_gemm_simt(ctx, st, en, spk_affine, e);
   }
-  fs->prompt_frames = prompt_frames;
-  fs->frames_done = 0;
-  fs->begun = true;
+  fs->prompt_frames[slot] = prompt_frames;
+  fs->frames_done[slot] = 0;
+  fs->begun[slot] = 1;
 }
 
-// tokens: device [n_tokens] = prompt tokens + every speech token so far INCLUDING the 3 look-ahead tokens (the same argument
-// the reference passes to flow.inference(streaming=True, finalize=False), cli/model.py:346-363).  Produces the mel frames that
-// call would return beyond those already delivered: rows [max(frames_done, prompt_frames), 2 * (n_tokens - 3)), written to
-// mel_out [*, 80]; returns their count.  Both chunk ends must be multiples of the 50-frame static chunk (the reference's hop
-// schedule guarantees it: cli/model.py:346-352 pads the first hop to the 25-token grid).
-int flow_stream_chunk(cvk_ctx* ctx, cvk_flow_stream* fs, const int32_t* tokens, int n_tokens, float* mel_out, int mel_cap_frames, cudaStream_t st) {
-  CVK_REQUIRE(fs->kind == 0 ? (ctx->flow && ctx->flow->tok_emb) : (ctx->dit && ctx->dit->tok_emb), "flow stage of this session not finalised");
+// B begun slots advance at once.  tokens: device, B prefixes back to back (token_lens[b] each) = prompt tokens + every speech
+// token so far INCLUDING the 3 look-ahead tokens (the argument the reference passes to flow.inference(streaming=True,
+// finalize=False), cli/model.py:346-363).  Produces, for every slot, the mel frames that call would return beyond those already
+// delivered: rows [max(frames_done, prompt_frames), 2 * (token_lens[b] - 3)), written back to back to mel_out [*, 80], their
+// counts in n_out[b].  Both chunk ends must be multiples of the 50-frame static chunk (the reference's hop schedule guarantees
+// it: cli/model.py:346-352 pads the first hop to the 25-token grid).  Every slot is checked before anything is launched, so a
+// refused call leaves all slots as they were.
+void flow_stream_chunk_batch(cvk_ctx* ctx, cvk_flow_stream* fs, int B, const int* slots, const int32_t* tokens, const int* token_lens,
+                             float* mel_out, int mel_cap_frames, int* n_out, cudaStream_t st) {
+  require_stage(ctx, fs);
   CVK_REQUIRE(ctx->flow && ctx->flow->noise, "cvk_cfm_set_noise has not been called");
   FlowModel* m = ctx->flow;          // holds the CFM noise for both estimator kinds
-  CVK_REQUIRE(fs->begun, "cvk_flow_stream_begin has not been called");
+  CVK_REQUIRE(B >= 1 && B <= fs->n_slots, "flow stream: bad batch size");
   const int CH = 2 * CHUNK_TOK;
-  const int T_total = 2 * (n_tokens - 3);
-  const int T_prev = fs->frames_done;
-  CVK_REQUIRE(T_total > T_prev, "flow stream: no new frames in this call");
-  CVK_REQUIRE(T_total % CH == 0 && T_prev % CH == 0, "flow stream: chunk ends must be multiples of the 50-frame static chunk");
-  CVK_REQUIRE(T_total <= fs->cap, "flow stream: cache capacity exceeded");
-  CVK_REQUIRE(fs->prompt_frames < T_total, "flow stream: prompt_feat longer than the generated mel");
-  const int n_new = T_total - T_prev;
-  const int skip = fs->prompt_frames > T_prev ? fs->prompt_frames - T_prev : 0;   // prompt rows are computed but not returned
-  CVK_REQUIRE(n_new - skip <= mel_cap_frames, "flow stream: output buffer too small");
+  std::vector<int> T_total(B), T_prev(B), n_new(B), skip(B), seen(fs->n_slots, 0);
+  int out_frames = 0, max_total = 0;
+  for (int b = 0; b < B; ++b) {
+    const int sl = slots[b];
+    CVK_REQUIRE(sl >= 0 && sl < fs->n_slots, "flow stream: slot out of range");
+    CVK_REQUIRE(!seen[sl], "flow stream: a slot appears twice in one call");
+    seen[sl] = 1;
+    CVK_REQUIRE(fs->begun[sl], "cvk_flow_stream_slot_begin has not been called for this slot");
+    T_total[b] = 2 * (token_lens[b] - 3);
+    T_prev[b] = fs->frames_done[sl];
+    CVK_REQUIRE(T_total[b] > T_prev[b], "flow stream: no new frames in this call");
+    CVK_REQUIRE(T_total[b] % CH == 0 && T_prev[b] % CH == 0, "flow stream: chunk ends must be multiples of the 50-frame static chunk");
+    CVK_REQUIRE(T_total[b] <= fs->cap, "flow stream: cache capacity exceeded");
+    CVK_REQUIRE(fs->prompt_frames[sl] < T_total[b], "flow stream: prompt_feat longer than the generated mel");
+    n_new[b] = T_total[b] - T_prev[b];
+    skip[b] = fs->prompt_frames[sl] > T_prev[b] ? fs->prompt_frames[sl] - T_prev[b] : 0;   // prompt rows are computed but not returned
+    out_frames += n_new[b] - skip[b];
+    max_total = std::max(max_total, T_total[b]);
+  }
+  CVK_REQUIRE(out_frames <= mel_cap_frames, "flow stream: output buffer too small");
+  CVK_REQUIRE(m->noise_T >= max_total, "the CFM noise tensor is too short");
   ctx->arena.reset();
   Seqs s2;
-  int lens_tok[1] = {n_tokens};
   Mat mu_full;
   if (fs->kind == 0) {
-    // encoder over the whole prefix (1.5 % of the flow FLOPs; its chunk mask + look-ahead make the prefix rows final as well)
-    Mat h = encoder_forward(ctx, st, tokens, lens_tok, 1, 1, 3, &s2);
+    // encoder over the whole prefixes (1.5 % of the flow FLOPs; its chunk mask + look-ahead make the prefix rows final as well)
+    Mat h = encoder_forward(ctx, st, tokens, token_lens, B, 1, 3, &s2);
     Mat ha = h;
     if (ctx->act_dtype != DT_F32) {
       ha = arena_mat(ctx, ctx->act_dtype, s2.R, D_ENC);
@@ -1371,28 +1433,47 @@ int flow_stream_chunk(cvk_ctx* ctx, cvk_flow_stream* fs, const int32_t* tokens, 
     e.out = mu_full;
     conv_gemm(ctx, st, ha, m->enc_proj, e);
   } else {
-    mu_full = dit_mu_forward(ctx, st, tokens, lens_tok, 1, 3, &s2);      // token embedding + look-ahead layer + x2 repeat: row-local
+    mu_full = dit_mu_forward(ctx, st, tokens, token_lens, B, 3, &s2);      // token embedding + look-ahead layer + x2 repeat: row-local
   }
-  CVK_REQUIRE(s2.len[0] == T_total, "flow stream: conditioning length mismatch");
-  // geometry of the new rows
-  int lens_new[1] = {n_new};
-  Seqs s1 = make_seqs(ctx, lens_new, 1, 8, 1, 0, st);
+  for (int b = 0; b < B; ++b) CVK_REQUIRE(s2.len[b] == T_total[b], "flow stream: conditioning length mismatch");
+  // geometry of the new rows; per-sequence inputs gathered from each slot's position
+  Seqs s1 = make_seqs(ctx, n_new.data(), B, 8, 1, 0, st);
   Mat mu = arena_mat(ctx, DT_F32, s1.R, N_MEL, N_MEL), cond = arena_mat(ctx, DT_F32, s1.R, N_MEL, N_MEL), x = arena_mat(ctx, DT_F32, s1.R, N_MEL, N_MEL);
+  Mat spk = arena_mat(ctx, DT_F32, B, N_MEL, N_MEL);
   zero_mat(ctx, st, mu); zero_mat(ctx, st, cond); zero_mat(ctx, st, x);
-  const size_t rowb = sizeof(float) * N_MEL;
-  CVK_CHECK_CUDA(cudaMemcpyAsync(mu.f32() + (size_t)s1.start[0] * N_MEL, mu_full.f32() + (size_t)(s2.start[0] + T_prev) * N_MEL, rowb * n_new,
-                                 cudaMemcpyDeviceToDevice, st));
-  if (skip > 0)
-    CVK_CHECK_CUDA(cudaMemcpyAsync(cond.f32() + (size_t)s1.start[0] * N_MEL, fs->prompt_feat + (size_t)T_prev * N_MEL, rowb * skip, cudaMemcpyDeviceToDevice, st));
-  CVK_REQUIRE(m->noise && m->noise_T >= T_total, "cvk_cfm_set_noise has not been called (or the noise tensor is too short)");
-  CVK_CHECK_CUDA(cudaMemcpyAsync(x.f32() + (size_t)s1.start[0] * N_MEL, m->noise + (size_t)T_prev * N_MEL, rowb * n_new, cudaMemcpyDeviceToDevice, st));
-  int geo[6] = {0, fs->cap, T_total, T_total, T_prev, T_prev};
-  int* d_tmp = upload(ctx, std::vector<int>(geo, geo + 6), st);
-  CVK_CHECK_CUDA(cudaMemcpyAsync(fs->d_geo, d_tmp, sizeof(int) * 6, cudaMemcpyDeviceToDevice, st));
-  cfm_solve_packed(ctx, st, s1, lens_new, mu, cond, fs->spk, x, fs->n_steps, 0.7f, 1, fs->kind, fs);
-  CVK_CHECK_CUDA(cudaMemcpyAsync(mel_out, x.f32() + (size_t)(s1.start[0] + skip) * N_MEL, rowb * (n_new - skip), cudaMemcpyDeviceToDevice, st));
-  fs->frames_done = T_total;
-  return n_new - skip;
+  std::vector<int> gi(3 * B);
+  for (int b = 0; b < B; ++b) {
+    gi[b] = T_prev[b];
+    gi[B + b] = fs->prompt_frames[slots[b]];
+    gi[2 * B + b] = slots[b];
+  }
+  {
+    const int* d_gi = upload(ctx, gi, st);
+    int bx = s1.max_len < 1024 ? s1.max_len : 1024;
+    stream_gather_kernel<<<dim3(bx, B), 96, 0, st>>>(mu_full.f32(), s2.d_start, m->noise, fs->prompt_feat, fs->spk, fs->cap, d_gi, B, s1.d_start,
+                                                     s1.d_len, mu.f32(), cond.f32(), x.f32(), spk.f32());
+    ctx->launches++;
+    CVK_LAUNCH_CHECK();
+  }
+  // cache geometry of the 2B CFG sequences: sequence b (conditional) and b + B (unconditional) of slot s use K/V rows from
+  // (2s + c) * cap and convolution state 2s + c
+  const int n2 = 2 * fs->n_slots;
+  std::vector<int> geo(4 * n2, 0);
+  for (int b2 = 0; b2 < 2 * B; ++b2) {
+    const int b = b2 % B, c = b2 / B, state = 2 * slots[b] + c;
+    geo[b2] = state * fs->cap;
+    geo[n2 + b2] = T_total[b];
+    geo[2 * n2 + b2] = T_prev[b];
+    geo[3 * n2 + b2] = state;
+  }
+  int* d_tmp = upload(ctx, geo, st);
+  CVK_CHECK_CUDA(cudaMemcpyAsync(fs->d_geo, d_tmp, sizeof(int) * geo.size(), cudaMemcpyDeviceToDevice, st));
+  cfm_solve_packed(ctx, st, s1, n_new.data(), mu, cond, spk.f32(), x, fs->n_steps, 0.7f, 1, fs->kind, fs);
+  unpack_rows_skip(ctx, st, x, s1, skip.data(), mel_out, N_MEL);
+  for (int b = 0; b < B; ++b) {
+    fs->frames_done[slots[b]] = T_total[b];
+    n_out[b] = n_new[b] - skip[b];
+  }
 }
 
 // ================================================================================================ CosyVoice3 entry points

@@ -57,6 +57,9 @@ SIGNATURES = {
     "cvk_flow_stream_bytes": (ctypes.c_longlong, [_vp]),
     "cvk_flow_stream_begin": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int, _vp, _vp]),
     "cvk_flow_stream_chunk": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int, _vp, ctypes.c_int, _c_int_p, _vp]),
+    "cvk_flow_stream_slots_create": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(_vp)]),
+    "cvk_flow_stream_slot_begin": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, ctypes.c_int, _vp, _vp]),
+    "cvk_flow_stream_chunk_batch": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _c_int_p, _vp, _c_int_p, _vp, ctypes.c_int, _c_int_p, _vp]),
     "cvk_cfm_set_noise": (ctypes.c_int, [_vp, _vp, ctypes.c_int, ctypes.c_int]),
     "cvk_hift3_set_noise": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_longlong, ctypes.c_int]),
     "cvk_hift3_inference": (ctypes.c_int, [_vp, _vp, _c_int_p, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp, _vp]),
@@ -378,6 +381,33 @@ class Context:
         n = ctypes.c_int(0)
         self._check(self.lib.cvk_flow_stream_chunk(self.h, fs, _ptr(tokens), int(tokens.numel()), _ptr(mel), cap, ctypes.byref(n), _stream()))
         return mel[:n.value]
+
+    def flow_stream_slots(self, n_slots, max_frames, n_timesteps=10, dit=False):
+        """One session holding n_slots utterances of up to max_frames mel frames each (cvk_flow_stream_slots_create)."""
+        s = ctypes.c_void_p()
+        self._check(self.lib.cvk_flow_stream_slots_create(self.h, int(bool(dit)), int(n_slots), int(max_frames), int(n_timesteps),
+                                                          ctypes.byref(s)))
+        return s
+
+    def flow_stream_slot_begin(self, fs, slot, prompt_feat, embedding):
+        """new utterance in `slot`: prompt_feat [Tp,80] (may be empty), embedding [192] or [1,192]"""
+        pf = _f32(prompt_feat, self.device) if prompt_feat is not None and prompt_feat.numel() else None
+        emb = _f32(embedding, self.device)
+        self._check(self.lib.cvk_flow_stream_slot_begin(self.h, fs, int(slot), _ptr(pf), 0 if pf is None else int(pf.shape[0]), _ptr(emb),
+                                                        _stream()))
+
+    def flow_stream_chunk_batch(self, fs, slots, tokens_list):
+        """Advance the distinct slots `slots` at once; tokens_list[b] = slot b's prompt tokens + speech tokens so far + 3
+        look-ahead tokens.  Returns (new mel frames of every slot back to back [sum n, 80] on the device, n list)."""
+        lens = [int(t.numel()) for t in tokens_list]
+        tokens = torch.cat([t.reshape(-1).to(dtype=torch.int32) for t in tokens_list]).to(self.device).contiguous()
+        cap = 2 * sum(lens)
+        mel = torch.empty(cap, 80, device=self.device)
+        n = (ctypes.c_int * len(lens))()
+        self._check(self.lib.cvk_flow_stream_chunk_batch(self.h, fs, len(lens), _ints(slots), _ptr(tokens), _ints(lens), _ptr(mel), cap, n,
+                                                         _stream()))
+        n = list(n)
+        return mel[:sum(n)], n
 
     # ------------------------------------------------------------------ LM
     def lm_session(self, max_batch, max_context):

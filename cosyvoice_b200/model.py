@@ -94,6 +94,7 @@ class B200CosyVoice2Model:
         self._lm_streams = []
         self.flow_stream_dict = {}           # uuid -> cvk_flow_stream handle, or False once a request has left the chunk grid
         self._idle_flow_streams = []
+        self._idle_slot_session = None       # ((dit, n_slots, cap), cvk_flow_stream handle) kept by tts_stream_batch
         self.lm_chains = 1                   # independent decode chains run concurrently (see lm_generate)
         self._window = torch.from_numpy(self.speech_window).float().to(self.device)
         self.n_timesteps = 10
@@ -240,7 +241,7 @@ class B200CosyVoice2Model:
                             c["left"] = int(((c["max_len_host"] - cnt) * (dn == 0)).max())
                 n += steps_per_sync
                 if on_progress is not None:
-                    on_progress(st[0]["out_ids"], st[0]["out_count"], st[0]["live"])
+                    on_progress(st[0]["out_ids"], st[0]["out_count"], st[0]["live"], st[0]["done"])
                 if all(c["live"] == 0 for c in st) or n > mx + steps_per_sync:
                     break
             out = [None] * B
@@ -547,23 +548,27 @@ class B200CosyVoice2Model:
 
         st = {"consumed": 0, "silent": 0}
 
-        def progress(out_ids, out_count, live):
-            n = int(out_count[0].item())
-            if n > st["consumed"]:
-                for tok in out_ids[0, st["consumed"]:n].tolist():
-                    if tok in self.silent_tokens:            # cli/model.py:121-127 (empty list for CosyVoice2: never taken)
-                        st["silent"] += 1
-                        if st["silent"] > 5:
-                            continue
-                    else:
-                        st["silent"] = 0
-                    self.tts_speech_token_dict[uuid].append(tok)
-                st["consumed"] = n
+        def progress(out_ids, out_count, live, done):
+            self._take_tokens(out_ids[0], int(out_count[0].item()), st, self.tts_speech_token_dict[uuid])
         # the LM job decodes on its own stream (cli/model.py:103: `with self.llm_context`, a side stream) while token2wav runs on
         # the model's stream
         self.lm_generate([text], [prompt_text], [llm_prompt_speech_token], steps_per_sync=8, on_progress=progress,
                          stream=self._new_lm_stream())
         self.llm_end_dict[uuid] = True
+
+    def _take_tokens(self, out_ids, n, st, dst):
+        """append ids [st["consumed"], n) of one LM row to dst, dropping silent tokens past 5 in a row (cli/model.py:121-127;
+        an empty list for CosyVoice2: never taken)"""
+        if n > st["consumed"]:
+            for tok in out_ids[st["consumed"]:n].tolist():
+                if tok in self.silent_tokens:
+                    st["silent"] += 1
+                    if st["silent"] > 5:
+                        continue
+                else:
+                    st["silent"] = 0
+                dst.append(tok)
+            st["consumed"] = n
 
     def vc_job(self, source_speech_token, uuid):
         self.tts_speech_token_dict[uuid] = source_speech_token.flatten().tolist()
@@ -617,3 +622,203 @@ class B200CosyVoice2Model:
             self.hift_cache_dict.pop(this_uuid)
         self._release_flow_stream(this_uuid)
         self.stream.synchronize()
+
+    # ---------------------------------------------------------------- batched streaming synthesis
+    def tts_stream_batch(self, inputs, uniforms=None):
+        """Streaming synthesis of several requests at once.  inputs: list of dicts with the kwargs of tts() (as for tts_batch);
+        uniforms: LM sampling uniforms [steps, len(inputs), 2] (default: drawn like tts_batch).  Returns a generator of
+        (i, {"tts_speech": float32 CPU [1, n]}, is_last).  Request i's chunks arrive in order and are what tts(stream=True) yields
+        for it alone on a fresh model instance: same hop schedule, same mel / source / speech caches, same hamming cross-fade,
+        same final non-streaming call.
+
+        One batched LM generation runs in a thread on its own stream.  Every round collects the requests whose token count
+        reached offset + hop + 3 and advances them together: ONE cvk_flow_stream_chunk_batch call on a multi-slot flow session
+        for those that can use a slot, ONE prefix-recompute flow call (the reference's schedule, cli/model.py:346-363) for the
+        rest (the rule of _flow_stream_chunk), then ONE vocoder call and ONE device-to-host copy for all of them.  Requests whose
+        LM has ended and whose remainder is below hop + 3 finish together in one non-streaming flow call and one vocoder call.
+
+        Differences from tts(stream=True): every request keeps its own hop (25, doubling up to token_max_hop_len), so
+        self.token_hop_len - which the reference keeps on the shared instance (cli/model.py:359-360) - is neither read nor
+        written.  Vocoder noise is drawn per request per chunk, in ascending request order within a round (noise_fn when set).
+        Text generators (text-streaming LM) and source_speech_token (voice conversion) inputs raise ValueError."""
+        for r in inputs:
+            if not torch.is_tensor(r.get("text")):
+                raise ValueError("tts_stream_batch: text must be a token tensor; text generators stream through tts()")
+            sst = r.get("source_speech_token")
+            if sst is not None and sst.shape[1] != 0:
+                raise ValueError("tts_stream_batch: source_speech_token (voice conversion) streams through tts()")
+        return self._stream_batch(list(inputs), uniforms)
+
+    def _stream_batch(self, inputs, uniforms):
+        B = len(inputs)
+        if B == 0:
+            return
+        toks = [[] for _ in range(B)]
+        ended = [False] * B
+        taken = [{"consumed": 0, "silent": 0} for _ in range(B)]
+        lm_err, lm_end = [], threading.Event()
+
+        def progress(out_ids, out_count, live, done):
+            cnt, dn, ids = out_count.tolist(), done.tolist(), out_ids.cpu()
+            for b in range(B):
+                self._take_tokens(ids[b], cnt[b], taken[b], toks[b])
+                if dn[b]:
+                    ended[b] = True                  # after its tokens: a reader that sees the flag sees every token
+
+        def lm_job():
+            try:
+                self.lm_generate([r["text"] for r in inputs], [r["prompt_text"] for r in inputs], [r["llm_prompt_speech_token"] for r in inputs],
+                                 uniforms, steps_per_sync=8, on_progress=progress, stream=self._new_lm_stream())
+            except BaseException as e:
+                lm_err.append(e)
+            finally:
+                lm_end.set()
+
+        hop0 = 25                                        # cosyvoice2.yaml static chunk, the first hop of every request
+        P = [int(r["flow_prompt_speech_token"].shape[1]) for r in inputs]
+        pad = [int(np.ceil(p / hop0) * hop0 - p) for p in P]
+        offset, hop, cache, finished = [0] * B, [hop0] * B, [None] * B, [False] * B
+        # rows that may use a session slot (prompt mel 2 frames per prompt token); one slot each, sized for the longest
+        slotted = [b for b in range(B) if self.incremental_flow and int(inputs[b]["prompt_speech_feat"].shape[1]) == TOKEN_MEL_RATIO * P[b]]
+        cap = max([min(self.stream_cache_frames, TOKEN_MEL_RATIO * (P[b] + int(inputs[b]["text"].shape[1] * self.max_token_text_ratio)))
+                   for b in slotted] + [2 * hop0])
+        sess = None
+        if slotted:
+            try:
+                sess = self._checkout_slots(len(slotted), cap)
+            except cvk.CvkError:
+                slotted = []                             # no memory for the caches: every request recomputes its prefixes
+        slot = {b: i for i, b in enumerate(slotted)}
+        lm = threading.Thread(target=lm_job, daemon=True)
+        lm.start()
+        try:
+            while not all(finished):
+                over = lm_end.is_set()
+                if lm_err:
+                    raise lm_err[0]
+                ready, fin = [], []
+                for b in range(B):
+                    if finished[b]:
+                        continue
+                    done = ended[b] or over              # read before the token count (see progress)
+                    need = hop[b] + (pad[b] if offset[b] == 0 else 0) + PRE_LOOKAHEAD
+                    if len(toks[b]) - offset[b] >= need:
+                        ready.append((b, toks[b][:offset[b] + need], need - PRE_LOOKAHEAD))
+                    elif done:
+                        fin.append(b)
+                if ready:
+                    mels = self._stream_round_mel(inputs, [(b, t) for b, t, _ in ready], offset, slot, sess)
+                    rows = [b for b, _, _ in ready]
+                    for (b, w) in zip(rows, self._stream_round_vocode(rows, mels, cache, False)):
+                        yield b, {"tts_speech": w}, False
+                    for b, _, this_hop in ready:
+                        offset[b] += this_hop
+                        hop[b] = min(self.token_max_hop_len, hop[b] * self.stream_scale_factor)
+                if fin:
+                    for b in fin:
+                        finished[b] = True
+                    rows = [b for b in fin if toks[b]]
+                    outs = {}
+                    if rows:
+                        mel, lens = self.flow_batch([torch.tensor(toks[b], dtype=torch.int32).unsqueeze(0) for b in rows],
+                                                    [inputs[b]["flow_prompt_speech_token"] for b in rows], [inputs[b]["prompt_speech_feat"] for b in rows],
+                                                    [inputs[b]["flow_embedding"] for b in rows], streaming=False, finalize=True)
+                        mels = [m[offset[b] * TOKEN_MEL_RATIO:] for b, m in zip(rows, torch.split(mel, lens, 0))]
+                        outs = dict(zip(rows, self._stream_round_vocode(rows, mels, cache, True)))
+                    for b in fin:
+                        yield b, {"tts_speech": outs.get(b, torch.zeros(1, 0))}, True
+                if not ready and not fin:
+                    time.sleep(0.005)
+        finally:
+            lm.join()
+            self._checkin_slots(sess)
+
+    def _stream_round_mel(self, inputs, rows, offset, slot, sess):
+        """new mel frames [n_b, 80] (device) of one round's rows (b, token prefix incl. look-ahead): ONE chunk_batch call for the
+        rows that can use their session slot, ONE prefix-recompute flow call for the others.  A row that leaves the slot rule
+        (chunk end off the 50-frame grid, over the slot capacity) recomputes from then on, like tts()."""
+        d = self.device
+        on_slot, other, new = [], [], {}
+        for b, t in rows:
+            P = int(inputs[b]["flow_prompt_speech_token"].shape[1])
+            total = TOKEN_MEL_RATIO * (P + len(t) - PRE_LOOKAHEAD)
+            done = TOKEN_MEL_RATIO * (P + offset[b]) if offset[b] else 0
+            if b in slot and total % 50 == 0 and done % 50 == 0 and total <= sess[0][2]:
+                on_slot.append((b, t))
+            else:
+                slot.pop(b, None)
+                other.append((b, t))
+        if on_slot:
+            with torch.cuda.stream(self.stream), self.ctx.lock:
+                fs = sess[1]
+                for b, _ in on_slot:
+                    if offset[b] == 0:
+                        r = inputs[b]
+                        self.ctx.flow_stream_slot_begin(fs, slot[b], r["prompt_speech_feat"][0].to(d, non_blocking=True),
+                                                        r["flow_embedding"].reshape(-1).to(d, non_blocking=True))
+                tl = [torch.cat([inputs[b]["flow_prompt_speech_token"].reshape(-1), torch.tensor(t, dtype=torch.int32)]).to(torch.int32)
+                      for b, t in on_slot]
+                mel, n = self.ctx.flow_stream_chunk_batch(fs, [slot[b] for b, _ in on_slot], tl)
+                new.update(zip([b for b, _ in on_slot], torch.split(mel, n, 0)))
+        if other:
+            mel, lens = self.flow_batch([torch.tensor(t, dtype=torch.int32).unsqueeze(0) for _, t in other],
+                                        [inputs[b]["flow_prompt_speech_token"] for b, _ in other], [inputs[b]["prompt_speech_feat"] for b, _ in other],
+                                        [inputs[b]["flow_embedding"] for b, _ in other], streaming=True, finalize=False)
+            for (b, _), m in zip(other, torch.split(mel, lens, 0)):
+                new[b] = m[offset[b] * TOKEN_MEL_RATIO:]
+        return [new[b] for b, _ in rows]
+
+    def _stream_round_vocode(self, rows, mels, cache, finalize):
+        """token2wav's vocoder half (cli/model.py:305-326) for one round's rows in ONE vocoder call (per-row cached mel frames
+        and cached source) and ONE device-to-host copy; updates the rows' caches.  Returns float32 CPU [1, n] per row."""
+        d = self.device
+        with torch.cuda.stream(self.stream):
+            tts_mels = [torch.cat([cache[b]["mel"], m], 0) if cache[b] is not None else m for b, m in zip(rows, mels)]
+            lens = [int(m.shape[0]) for m in tts_mels]
+            cached = [b for b in rows if cache[b] is not None]
+            cs = torch.cat([cache[b]["source"] for b in cached]) if cached else None
+            cl = [int(cache[b]["source"].shape[0]) if cache[b] is not None else 0 for b in rows] if cached else None
+            mel = torch.cat(tts_mels, 0).contiguous()
+            with self.lock:                              # one device generator shared by the request threads
+                noise = torch.cat([self.noise_fn(L * SAMPLES_PER_FRAME).to(d) if self.noise_fn is not None
+                                   else torch.randn(L * SAMPLES_PER_FRAME, 9, device=d, generator=self.generator) for L in lens])
+        wav, src = self.hift_batch(mel, lens, cs, cl, noise=noise)
+        with torch.cuda.stream(self.stream):
+            outs, o = [], 0
+            for b, tm, L in zip(rows, tts_mels, lens):
+                w, s = wav[o:o + L * SAMPLES_PER_FRAME], src[o:o + L * SAMPLES_PER_FRAME]
+                o += L * SAMPLES_PER_FRAME
+                if cache[b] is not None:
+                    w = self._fade_in_out(w, cache[b]["speech"])
+                if not finalize:
+                    cache[b] = {"mel": tm[-self.mel_cache_len:].clone(), "source": s[-self.source_cache_len:].clone(),
+                                "speech": w[-self.source_cache_len:].clone()}
+                    w = w[:-self.source_cache_len]
+                outs.append(w)
+            host = torch.cat(outs).cpu()                 # one D2H for the round
+        self.stream.synchronize()
+        return [c.unsqueeze(0) for c in torch.split(host, [int(w.shape[0]) for w in outs])]
+
+    def _checkout_slots(self, n_slots, cap):
+        """a multi-slot flow session ((dit, n_slots, cap), handle) with at least n_slots slots of cap frames: the idle one when it
+        is large enough, else a new one (cvk.CvkError when there is no memory for it)"""
+        with self._pool_lock:
+            idle, self._idle_slot_session = self._idle_slot_session, None
+        if idle is not None:
+            (dit, n, c), fs = idle
+            if dit == self.flow_stream_dit and n >= n_slots and c >= cap:
+                return idle
+            self.stream.synchronize()
+            self.ctx.flow_stream_destroy(fs)
+        with torch.cuda.stream(self.stream), self.ctx.lock:
+            return (self.flow_stream_dit, n_slots, cap), self.ctx.flow_stream_slots(n_slots, cap, self.n_timesteps, dit=self.flow_stream_dit)
+
+    def _checkin_slots(self, sess):
+        """keep one idle multi-slot session for the next call; a previously idle one is destroyed"""
+        if sess is None:
+            return
+        self.stream.synchronize()
+        with self._pool_lock:
+            old, self._idle_slot_session = self._idle_slot_session, sess
+        if old is not None:
+            self.ctx.flow_stream_destroy(old[1])

@@ -78,3 +78,8 @@ class B200CosyVoice3Model(B200CosyVoice2Model):
             wav = wav[cache["speech_offset"]:]
             cache["speech_offset"] += wav.shape[0]
         return wav.unsqueeze(0)
+
+    def tts_stream_batch(self, inputs, uniforms=None):
+        """Not available for CosyVoice3: its token2wav keeps every mel frame and re-runs the causal vocoder over them, a different
+        schedule from the CosyVoice2 caches that B200CosyVoice2Model.tts_stream_batch batches.  Stream through tts()."""
+        raise NotImplementedError("tts_stream_batch is CosyVoice2 only; CosyVoice3 streams through tts(stream=True)")

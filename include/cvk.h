@@ -19,8 +19,8 @@
  *    concurrently with workspace calls and with each other on DISTINCT sessions and streams - this is the reference's
  *    own concurrency (LM side thread + side stream next to token2wav, cli/model.py:101-129, 268; several requests in
  *    flight, runtime/python/grpc/server.py:69).  One session is never used by two host threads at once.  Streaming-flow
- *    sessions (cvk_flow_stream_*) hold caches only: their begin / chunk calls use the workspace and are serialised like every
- *    other flow call.
+ *    sessions (cvk_flow_stream_*, one slot or several) hold caches only: their begin / chunk / chunk_batch calls use the
+ *    workspace and are serialised like every other flow call.
  *  - Return value: 0 on success, a negative cvk_status otherwise; cvk_last_error(ctx) holds the message.  No C++
  *    exception crosses the ABI.  There is NO CPU fallback: without a CUDA device cvk_create fails.
  */
@@ -166,6 +166,27 @@ int cvk_flow_stream_begin(cvk_ctx* ctx, cvk_flow_stream* fs, const float* prompt
                           void* stream);
 int cvk_flow_stream_chunk(cvk_ctx* ctx, cvk_flow_stream* fs, const int32_t* tokens, int n_tokens, float* mel_out,
                           int mel_capacity_frames, int* n_frames_out, void* stream);
+
+/* ---- batched streaming flow: one session, several utterances ----------------------------------------------------------------
+ * The reference serves concurrent streams one thread each, every chunk its own flow.inference call (cli/model.py:343-363).  A
+ * multi-slot session holds n_slots utterances in one allocation (slot s, CFG branch c caches K/V rows from (2s + c) * cap), and
+ * ONE chunk_batch call advances B distinct begun slots through one encoder / estimator pass, so B streams cost one chunk's
+ * launches.  Slots in one call may sit at different chunk positions and have different prompt lengths and chunk lengths.
+ * slots_create: kind 0 = CosyVoice2 U-Net (stage "flow"), 1 = CosyVoice3 DiT (stage "flow3"); max_frames per slot;
+ * cvk_flow_stream_bytes reports the whole allocation.  cvk_flow_stream_create / cvk_flow3_stream_create are n_slots = 1,
+ * cvk_flow_stream_begin is slot 0 and cvk_flow_stream_chunk a batch of one.
+ * slot_begin: new utterance in `slot` (same arguments as cvk_flow_stream_begin).
+ * chunk_batch: slots_host [B] distinct begun slots; tokens = the B token prefixes back to back (token_lens_host[b] each: prompt +
+ * speech so far + 3 look-ahead, as for cvk_flow_stream_chunk); mel_out receives the new frames of every slot back to back
+ * ([sum n_frames_out_host[b], 80], the ragged ABI convention), n_frames_out_host[b] their counts.  Every slot is checked (in
+ * range, distinct, begun, both chunk ends on the 50-frame grid, capacity, mel_capacity_frames) before anything is launched: a
+ * refused call returns CVK_ERR_INVALID and leaves every slot's state unchanged. */
+int cvk_flow_stream_slots_create(cvk_ctx* ctx, int kind, int n_slots, int max_frames, int n_timesteps, cvk_flow_stream** out);
+int cvk_flow_stream_slot_begin(cvk_ctx* ctx, cvk_flow_stream* fs, int slot, const float* prompt_feat, int prompt_frames,
+                               const float* embedding, void* stream);
+int cvk_flow_stream_chunk_batch(cvk_ctx* ctx, cvk_flow_stream* fs, int B, const int* slots_host, const int32_t* tokens,
+                                const int* token_lens_host, float* mel_out, int mel_capacity_frames, int* n_frames_out_host,
+                                void* stream);
 
 /* ---- CosyVoice3 vocoder (stage "hift3") ------------------------------------------------------------------------------------
  * cosyvoice/hifigan/generator.py:572-726 CausalHiFTGenerator (+ f0_predictor.py:60-103 in float64, generator.py:716-717).
